@@ -2,7 +2,7 @@
 """bench.py — proofs/s on the BASELINE.json workload (Groth16, BN254, domain 2^20 synthetic chain circuit).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--log-n 20] [--impl reference]
-                    [--workload groth16|plonk|fflonk] [--curve bn128|bls12381]
+                    [--workload groth16|plonk|fflonk] [--curve bn128|bls12381] [--dump-outputs DIR]
 
 One step = one proof.  N = 1: the whole prover on one B200.  N > 1 (torchrun, one rank per GPU): every MSM is sharded
 by point range across the ranks (north star / SURVEY §8e) and the three A/B/C transform chains run on different ranks;
@@ -45,7 +45,14 @@ def parse():
     ap.add_argument("--witness-like", action="store_true", help="witness distribution of real circuits (SURVEY 8d): 50%% zeros, 25%% ones, 25%% uniform")
     ap.add_argument("--tune", action="append", default=[], help="experimental kernel-variant switch k=v (sb_set_tuning), e.g. 1=1 = legacy bucket reduction")
     ap.add_argument("--mode", default="shard", choices=["shard", "replicas"], help="N > 1: which number is `value` (the other one is reported beside it)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the proof of the last timed step to DIR/proof.npy (B200 arm)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the B200 arm's outputs; the reference arm has none to write")
+    return a
 
 
 # ------------------------------------------------------------------------------------------------ clocks sampler
@@ -110,6 +117,16 @@ def host_cores() -> int:
 def proof_hash(proof_obj) -> str:
     """sha256 of the canonical JSON text of the proof object (SURVEY §8c: proof.json text identical)."""
     return hashlib.sha256(json.dumps(proof_obj, sort_keys=True, separators=(",", ":")).encode()).hexdigest()
+
+
+def dump_outputs(out_dir: str | None, proof: np.ndarray) -> None:
+    """--dump-outputs: the proof bytes a prove call returns (affine points and field elements in the library's Montgomery
+    form), one float64 per byte so that the values are exact.  The inputs are fixed by the flags, so two builds given the
+    same flags must write the same file."""
+    if not out_dir:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "proof.npy"), np.asarray(proof, np.uint8).astype(np.float64))
 
 
 def golden_hash(workload: str, curve: str, L: int, witness_like: bool):
@@ -268,6 +285,7 @@ def run_b200(args):
         # per-stage breakdown of the last e2e step (CUDA events on the library's stream)
         brk = {"h2d_witness": curve.last_ms(1), "device_total": curve.last_ms(0)}
         dt_res = timed(lambda: step(True), args.steps)
+        proof_res = proof.copy()
     clocks = cs.summary()
     replicas = None
     if world > 1:
@@ -392,6 +410,7 @@ def run_b200(args):
         except Exception as e:  # the baseline is a report, never a reason to lose the GPU number
             line["cpu_baseline"] = {"error": str(e)}
     print(json.dumps(line))
+    dump_outputs(args.dump_outputs, proof_res)
     pk.release()
     curve.terminate()
     if dist is not None:

@@ -14,10 +14,12 @@ in tests/test_py_mirror.py), so at N = 1 the B200 proof is compared with it byte
 from __future__ import annotations
 
 import ctypes
+import functools
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import time
 
 import numpy as np
@@ -43,17 +45,15 @@ def _proof_bytes(proto: str, n8q: int) -> int:
 
 
 # ------------------------------------------------------------------------------------------------ CPU port (reference arm)
+@functools.lru_cache(maxsize=None)
 def host_flow_lib(proto: str):
-    """tests/host/host_<proto>.cpp compiled with OpenMP (cached under tests/host/build/)."""
+    """tests/host/host_<proto>.cpp compiled with OpenMP, once per process, in a temporary directory: the source tree may be
+    read-only, and a -march=native build must not be reused on another host."""
     src = os.path.join(ROOT, "tests", "host", f"host_{proto}.cpp")
-    out_dir = os.path.join(ROOT, "tests", "host", "build")
-    os.makedirs(out_dir, exist_ok=True)
-    so = os.path.join(out_dir, f"libhost{proto}_omp.so")
-    deps = [src, os.path.join(ROOT, "tests", "host", "host_backend.h")] + [os.path.join(ROOT, "snarkjs_b200", "csrc", f) for f in
-                                                                             ("plonk_flow.h", "plonk.cuh", "fflonk_flow.h", "fflonk.cuh", "fp.cuh")]
-    if not os.path.exists(so) or any(os.path.getmtime(d) > os.path.getmtime(so) for d in deps):
+    with tempfile.TemporaryDirectory(prefix="snarkjs_b200_host_") as tmp:
+        so = os.path.join(tmp, f"libhost{proto}_omp.so")
         subprocess.check_call(["g++", "-O3", "-march=native", "-fopenmp", "-std=c++17", "-shared", "-fPIC", "-o", so, src, "-ldl"])
-    lib = ctypes.CDLL(so)
+        lib = ctypes.CDLL(so)     # stays mapped after the file is removed
     fn = getattr(lib, f"hp_{proto}_prove")
     fn.restype = ctypes.c_int
     fn.argtypes = [ctypes.c_char_p, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_char_p, ctypes.c_void_p, ctypes.c_char_p, ctypes.c_int]
@@ -146,7 +146,7 @@ def run_b200(args):
     import snarkjs_b200
     from snarkjs_b200 import fflonk, plonk, synth
     from snarkjs_b200.curve import _ptr
-    from bench import ClockSampler, host_cores, proof_hash
+    from bench import ClockSampler, dump_outputs, host_cores, proof_hash
 
     proto, cname, L = args.workload, _curve_name(args), args.log_n
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -296,6 +296,7 @@ def run_b200(args):
         except Exception as e:
             line["cpu_baseline"] = {"error": str(e)}
     print(json.dumps(line))
+    dump_outputs(args.dump_outputs, proof)
     pk.release()
     curve.terminate()
     if dist is not None:

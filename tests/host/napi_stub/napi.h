@@ -98,12 +98,15 @@ class AsyncWorker {
     virtual ~AsyncWorker() {}
     Napi::Env Env() const { return Napi::Env(); }
     void SetError(const std::string& m) { err_ = m; failed_ = true; }
-    void Queue() { Execute(); if (failed_) OnError(Error::New(Env(), err_)); else OnOK(); delete this; }
+    // Execute() and the completion callback run at once, but the worker is only deleted at exit: node-addon-api deletes it
+    // after the completion callback, on a later turn of the event loop, so a binding may still read it after Queue().
+    void Queue() { Execute(); if (failed_) OnError(Error::New(Env(), err_)); else OnOK(); completed().emplace_back(this); }
  protected:
     virtual void Execute() = 0;
     virtual void OnOK() {}
     virtual void OnError(const Error&) {}
  private:
+    static std::vector<std::unique_ptr<AsyncWorker>>& completed() { static std::vector<std::unique_ptr<AsyncWorker>> w; return w; }
     std::string err_; bool failed_ = false;
 };
 }  // namespace Napi
