@@ -345,6 +345,8 @@ void prof_end(sb_ctx* c) {
         const int g = c->stats.tag[i / 2];
         if (g == PROF_ACC_G1) { c->stat[0] += ms; c->stat[2] += 1; c->stat[9] += ms; }
         else if (g == PROF_ACC_G2) { c->stat[1] += ms; c->stat[3] += 1; c->stat[10] += ms; }
+        else if (g == PROF_PAIR_G1) { c->stat[0] += ms; c->stat[9] += ms; }
+        else if (g == PROF_PAIR_G2) { c->stat[1] += ms; c->stat[10] += ms; }
         else if (g == PROF_SORT) c->stat[8] += ms;
         else if (g >= PROF_FOLD && g <= PROF_JOIN) c->stat[11 + (g - PROF_FOLD)] += ms;
     }

@@ -18,6 +18,7 @@
 //                 then a shared-memory tree to one point per window
 //   host          Horner over the W window sums (W*c doublings on 1 point: latency-bound, CPU is faster)
 #pragma once
+#include <algorithm>
 #include <cuda_runtime.h>
 #include "ec.cuh"
 #include "msm_geom.h"
@@ -29,6 +30,25 @@ static constexpr int MSM_ACC_THREADS = 128;
 static constexpr int MSM_RED_CHUNK = 16;    // buckets per thread in k_reduce
 static constexpr uint32_t MSM_INVALID_KEY = 0xffffffffu;
 static constexpr int MSM_COUNTS_SEG = 8;      // counts[8]: sorted entries per k_accumulate thread (counts[0] = valid entries, [1..7] = fold level sizes)
+
+// counts[] of a sorted list of M valid entries (one device thread): the entries per accumulation thread, target T, fitted so
+// that the grid is a whole number of waves of `wave` resident threads (MsmSorted comment; wave = 0: T as is), and the
+// level sizes of the fold cascade: level 0 always emits ceil(M/seg) heads; a level >= 1 with <= MSM_SEG inputs is the
+// last one (single thread, everything folded into the buckets) and emits none.
+__device__ inline void msm_fill_counts(uint64_t* out, uint64_t M, uint32_t T, uint32_t seg_lo, uint64_t wave) {
+    out[0] = M;
+    uint64_t seg = T;
+    if (wave) {
+        const uint64_t k = (M + wave * T - 1) / (wave * T);              // waves at the target size
+        if (k && k <= 3) seg = (M + k * wave - 1) / (k * wave);       // with 4+ waves the partial last wave still saturates the pipe (measured: no gain, more heads)
+        if (seg < seg_lo) seg = seg_lo;
+        if (seg > T) seg = T;
+    }
+    out[MSM_COUNTS_SEG] = seg;
+    uint64_t m = (M + seg - 1) / seg;
+    out[1] = m;
+    for (int l = 2; l < 8; l++) { m = (m <= MSM_SEG) ? 0 : (m + MSM_SEG - 1) / MSM_SEG; out[l] = m; }
+}
 
 
 // Window-size choice.  Cost model: W_eff*n mixed adds (10 modmul) + one pass over the buckets (~60 modmul each);
@@ -626,7 +646,9 @@ struct MsmLaunchStats {
     // optional profiling: event pairs recorded around kernel groups (tag = PROF_* below; accumulation uses cur_tag)
     cudaEvent_t* ev = nullptr; int nev = 0; int used = 0; int tag[128] = {0}; int cur_tag = 0;
 };
-enum { PROF_ACC_G1 = 1, PROF_ACC_G2 = 2, PROF_SORT = 3, PROF_FOLD = 4, PROF_REDUCE = 5, PROF_QAP = 6, PROF_NTT = 7, PROF_JOIN = 8 };
+// PROF_PAIR_G1/G2: batched-affine rounds, counted as accumulation time of the group but not as an accumulation launch
+enum { PROF_ACC_G1 = 1, PROF_ACC_G2 = 2, PROF_SORT = 3, PROF_FOLD = 4, PROF_REDUCE = 5, PROF_QAP = 6, PROF_NTT = 7, PROF_JOIN = 8,
+       PROF_PAIR_G1 = 9, PROF_PAIR_G2 = 10 };
 // one event pair around a group of launches on `st`; a no-op unless profiling is armed (api.cu prof_begin)
 struct ProfScope {
     MsmLaunchStats* s; cudaStream_t st; int idx = -1;
@@ -653,15 +675,30 @@ struct MsmSorted {
     uint32_t seg_lo = MSM_SEG;
 };
 
-// msm_sort.cu: helpers of the pairing rounds (non-template part)
-size_t msm_pair_scan_tmp_bytes(uint32_t NB);
-int msm_pair_offsets(const uint32_t* keys, const uint64_t* counts, uint32_t NB, uint32_t* off, cudaStream_t stream);
-int msm_pair_next_offsets(const uint32_t* off_in, uint32_t NB, uint32_t* sizes, uint32_t* off_out, void* tmp, size_t tmp_bytes, cudaStream_t stream);
-int msm_pair_counts(const uint32_t* off, uint32_t NB, uint64_t* counts, cudaStream_t stream);
+// msm_sort.cu: SM count of the current device, output positions of a batched-affine round (non-template part)
+int msm_sm_count();
+size_t msm_pair_scan_tmp_bytes(uint64_t items);
+int msm_pair_scan(const uint32_t* counts, uint32_t* pos, uint64_t items, void* tmp, size_t tmp_bytes, cudaStream_t stream);
 
 // msm_sort.cu: digits + radix sort + valid count.  d_scalars is a device pointer.
 int msm_sort_entries(const uint8_t* d_scalars, uint32_t sbytes, uint64_t n, MsmGeom g, MsmScratch& scratch,
                      cudaStream_t stream, MsmSorted* out, MsmLaunchStats* stats);
+
+// Scratch layout of msm_buckets_impl (byte offsets from its scratch_off) for a list of at most `total` entries.
+struct MsmBucketLayout { uint64_t heads0 = 0; size_t headsA = 0, hkA = 0, headsB = 0, hkB = 0, hkM = 0, part = 0, bytes = 0; };
+template <class F>
+MsmBucketLayout msm_bucket_layout(const MsmGeom& g, uint64_t total, uint32_t seg_lo) {
+    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
+    MsmBucketLayout L;
+    L.heads0 = (total + seg_lo - 1) / seg_lo;   // upper bound; the device knows the exact count (counts[1])
+    const uint64_t heads1 = (L.heads0 + MSM_SEG - 1) / MSM_SEG;
+    L.headsA = al((uint64_t)g.windows() * g.B * sizeof(XYZZ<F>)); L.hkA = L.headsA + al(L.heads0 * sizeof(XYZZ<F>));
+    L.headsB = L.hkA + al(L.heads0 * 4); L.hkB = L.headsB + al(heads1 * sizeof(XYZZ<F>));
+    L.hkM = L.hkB + al(heads1 * 4);                       // level-1 keys after the short-run fast path
+    L.part = L.hkM + al(L.heads0 * 4);
+    L.bytes = L.part + al(msm_reduce_scratch_elems(g) * sizeof(XYZZ<F>));
+    return L;
+}
 
 // Bucket accumulation + reduction for one base set.  Writes g.W window sums to d_wsum (device).  Asynchronous.
 // If tail_stream differs from stream, the throughput-bound accumulation runs on `stream` and the latency-bound tail
@@ -671,76 +708,88 @@ template <class F>
 int msm_buckets_impl(const Affine<F>* d_bases, const MsmSorted& s, MsmScratch& scratch, size_t scratch_off, cudaStream_t stream,
                      XYZZ<F>* d_wsum, MsmLaunchStats* stats, cudaStream_t tail_stream, cudaEvent_t ev_acc);
 
-// Entry: optional batched-affine pairing rounds (msm_pair.cuh) shrink the entry list first, then the segmented XYZZ
-// pipeline runs on what is left.  EXPERIMENTAL, off by default (enable with sb_set_tuning(4, 2), cap the rounds with
-// sb_set_tuning(5, R)): measured on B200 at 2^20 the rounds run the integer pipe at 40-60 % (scan + shared inversion +
-// two gather passes) against 93 % / 71 % for the XYZZ accumulation, which cancels the 6-vs-10 modmul advantage
-// (G1 3.7 ms vs 3.4 ms per MSM, G2 11.6 ms vs 11.8 ms; profiles/README.md).
+// Entry: batched-affine rounds (msm_pair.cuh) shrink the sorted list first where they pay, then the segmented XYZZ
+// pipeline runs on what is left.  The rounds are the default for BN254 G2 (an XYZZ mixed addition costs 27.5
+// modmul-equivalents there) on lists of >= PAIR_MIN_ENTRIES entries that average more than PAIR_STOP_DENSITY entries per
+// bucket (precomputed-table MSMs: 26 or more per bucket).  Measured on a B200
+// (1000 W), one registered 2^20 BN254 MSM, uniform scalars (profiles/ab_batch_affine.py, profiles/README.md):
+//   G2: XYZZ only 10.18 ms, 1 round 9.30, 2 rounds 8.96, 3 rounds 9.02, 4 rounds 9.23 -> stop at ~8 entries per bucket;
+//   G1: XYZZ only 3.24 ms, 1 round 3.39, 2 rounds 3.49 -> the rounds stay off (9.5 modmul per XYZZ addition is too
+//   close to the ~6 of an affine one plus the extra passes over memory).  BLS12-381 G2 has not been measured: off.
+// sb_set_tuning(4, 2) forces the rounds (at least one, and down to PAIR_FORCED_STOP_DENSITY), (4, 1) turns them off,
+// (5, R) caps their number.
+static constexpr double PAIR_STOP_DENSITY = 8.0;     // rounds run while the list averages more entries per bucket than this
+static constexpr double PAIR_FORCED_STOP_DENSITY = 2.0;
+static constexpr uint64_t PAIR_MIN_ENTRIES = 1ull << 20;
+static constexpr int PAIR_MAX_ROUNDS = 8;
+static constexpr uint64_t PAIR_MAX_SLOTS = 64;       // pair slots per thread
+template <class F> struct PairDefault { static constexpr bool value = false; };
+template <> struct PairDefault<Fp2<BnFq>> { static constexpr bool value = true; };
+
 template <class F>
 int msm_buckets(const Affine<F>* d_bases, const MsmSorted& s, MsmScratch& scratch, cudaStream_t stream,
                 XYZZ<F>* d_wsum, MsmLaunchStats* stats, cudaStream_t tail_stream = nullptr, cudaEvent_t ev_acc = nullptr) {
     const MsmGeom g = s.g;
-    const uint64_t NBl = (uint64_t)g.windows() * g.B;
-    const double avg = NBl ? (double)s.total / (double)NBl : 0.0;
-    if (g_msm_tuning[4] != 2 || avg < 4.0 || NBl >= (1ull << 31) || s.total >= (1ull << 31))
+    const uint64_t NB = (uint64_t)g.windows() * g.B;
+    const int mode = g_msm_tuning[4];
+    const double stop = mode == 2 ? PAIR_FORCED_STOP_DENSITY : PAIR_STOP_DENSITY;
+    const bool dense = NB && (double)s.total > PAIR_STOP_DENSITY * (double)NB;
+    const bool use = mode == 2 || (mode == 0 && PairDefault<F>::value && s.total >= PAIR_MIN_ENTRIES && dense);
+    if (!use || s.total == 0 || NB >= (1ull << 31) || s.total >= (1ull << 31))
         return msm_buckets_impl<F>(d_bases, s, scratch, 0, stream, d_wsum, stats, tail_stream, ev_acc);
-    const uint32_t NB = (uint32_t)NBl;
-    int R = 1; while ((1u << R) < 2.0 * avg && R < 8) R++;
-    if (g_msm_tuning[5] > 0 && g_msm_tuning[5] < R) R = g_msm_tuning[5];   // cap on the number of pairing rounds (experiments)
+    // Round plan on host upper bounds (the device knows the exact lengths): a round turns n entries into at most
+    // ceil(n/2) + (key changes) <= ceil(n/2) + min(NB, n); it is expected to leave n/2 + NB/2 (half the buckets end on an
+    // odd position).  Every round gets ~2048 threads per SM (several waves of both round kernels) and 1..64 slots per thread.
+    uint64_t ub[PAIR_MAX_ROUNDS + 1], Jub[PAIR_MAX_ROUNDS], T[PAIR_MAX_ROUNDS]; uint32_t K[PAIR_MAX_ROUNDS];
+    const uint64_t target = (uint64_t)msm_sm_count() * 2048;
+    double est = (double)s.total;
+    int R = 0; ub[0] = s.total;
+    while (R < PAIR_MAX_ROUNDS && (est > stop * (double)NB || (R == 0 && mode == 2))) {
+        Jub[R] = (ub[R] + 1) / 2;
+        uint64_t k = (Jub[R] + target) / target; if (k > PAIR_MAX_SLOTS) k = PAIR_MAX_SLOTS;
+        K[R] = (uint32_t)k;
+        T[R] = ((Jub[R] + k) / k + PAIR_THREADS - 1) / PAIR_THREADS * PAIR_THREADS;    // K * T >= Jub + 1 slots
+        ub[R + 1] = std::min(ub[R], (ub[R] + 1) / 2 + std::min(NB, ub[R]));
+        est = est / 2 + (double)NB / 2;
+        R++;
+    }
+    if (g_msm_tuning[5] > 0 && g_msm_tuning[5] < R) R = g_msm_tuning[5];
+    uint64_t Tmax = 0; for (int r = 0; r < R; r++) Tmax = std::max(Tmax, T[r]);
     auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
-    const uint64_t ub1 = (s.total + NB + 1) / 2;
-    const size_t scan_tmp = msm_pair_scan_tmp_bytes(NB);
-    const uint64_t pthreads = ((ub1 + PAIR_K - 1) / PAIR_K + PAIR_THREADS - 1) / PAIR_THREADS * PAIR_THREADS;
-    size_t o_offA = 0, o_offB = o_offA + al((size_t)(NB + 1) * 4), o_sizes = o_offB + al((size_t)(NB + 1) * 4);
-    size_t o_tmp = o_sizes + al((size_t)(NB + 1) * 4), o_cnt = o_tmp + al(scan_tmp);
-    size_t o_PA = o_cnt + 256, o_PB = o_PA + al(ub1 * sizeof(Affine<F>)), o_KA = o_PB + al(ub1 * sizeof(Affine<F>));
-    size_t o_KB = o_KA + al(ub1 * 4), o_L = o_KB + al(ub1 * 4), o_rest = o_L + al(pthreads * PAIR_K * sizeof(F));
-    // size the rest (buckets, heads, partials) for the list that survives the rounds
-    uint64_t ub = s.total; for (int r = 0; r < R; r++) ub = (ub + NB + 1) / 2;
-    MsmSorted s2 = s; s2.total = ub; s2.vals = nullptr; s2.seg_lo = MSM_SEG;
-    // first call sizes the whole scratch: probe the tail's requirement with a dry computation (same formula as impl)
-    {
-        const uint64_t heads0 = (ub + MSM_SEG - 1) / MSM_SEG, heads1 = (heads0 + MSM_SEG - 1) / MSM_SEG;
-        const uint32_t L = g.B < (uint32_t)MSM_RED_CHUNK ? g.B : MSM_RED_CHUNK;
-        const uint32_t ctas_per_window = (g.B / L + 127) / 128;
-        size_t need = al(NBl * sizeof(XYZZ<F>)) + al(heads0 * sizeof(XYZZ<F>)) + al(heads0 * 4) + al(heads1 * sizeof(XYZZ<F>)) + al(heads1 * 4) +
-                      al(heads0 * 4) + al(msm_reduce_scratch_elems(g) * sizeof(XYZZ<F>));
-        need += need / 8 + (1u << 20);   // margin: the impl must never grow (= reallocate) the scratch the rounds are using
-        if (!scratch.get(o_rest + need)) return (int)cudaErrorMemoryAllocation;
-    }
+    const size_t scan_tmp = msm_pair_scan_tmp_bytes(Jub[0] + 1);
+    const size_t o_outc = al((size_t)R * 128), o_pos = o_outc + al((Jub[0] + 1) * 4), o_tmp = o_pos + al((Jub[0] + 1) * 4);
+    const size_t o_pre = o_tmp + al(scan_tmp), o_tp = o_pre + al(Jub[0] * sizeof(F)), o_inv = o_tp + al(Tmax * sizeof(F));
+    const size_t o_P0 = o_inv + al(Tmax * sizeof(F)), o_P1 = o_P0 + al(ub[1] * sizeof(Affine<F>)), o_K0 = o_P1 + al(ub[1] * sizeof(Affine<F>));
+    const size_t o_K1 = o_K0 + al(ub[1] * 4), o_rest = o_K1 + al(ub[1] * 4);
+    MsmSorted s2 = s; s2.total = ub[R]; s2.vals = nullptr; s2.seg_lo = MSM_SEG / 2;       // k_pair_invert's count fit
+    // one allocation for the rounds and the pipeline behind them: the scratch must not be reallocated while the rounds use it
+    if (!scratch.get(o_rest + msm_bucket_layout<F>(g, s2.total, s2.seg_lo).bytes)) return (int)cudaErrorMemoryAllocation;
     uint8_t* base = (uint8_t*)scratch.p;
-    uint32_t* offA = (uint32_t*)(base + o_offA); uint32_t* offB = (uint32_t*)(base + o_offB); uint32_t* sizes = (uint32_t*)(base + o_sizes);
-    uint64_t* counts2 = (uint64_t*)(base + o_cnt);
-    Affine<F>* P[2] = {(Affine<F>*)(base + o_PA), (Affine<F>*)(base + o_PB)};
-    uint32_t* K[2] = {(uint32_t*)(base + o_KA), (uint32_t*)(base + o_KB)};
-    F* Ls = (F*)(base + o_L);
+    uint32_t* outc = (uint32_t*)(base + o_outc); uint32_t* pos = (uint32_t*)(base + o_pos);
+    F* pre = (F*)(base + o_pre); F* tprod = (F*)(base + o_tp); F* invp = (F*)(base + o_inv);
+    Affine<F>* P[2] = {(Affine<F>*)(base + o_P0), (Affine<F>*)(base + o_P1)};
+    uint32_t* Kb[2] = {(uint32_t*)(base + o_K0), (uint32_t*)(base + o_K1)};
+    const uint64_t wave = (uint64_t)msm_sm_count() * 4 * MSM_ACC_THREADS;
     int launches = 0;
-    ProfScope prof(stats, stats ? stats->cur_tag : 0, stream);
-    int rc = msm_pair_offsets(s.keys, s.counts, NB, offA, stream); launches++;
-    if (rc) return rc;
-    const Affine<F>* src = d_bases; uint32_t* in = offA; uint32_t* out = offB;
-    uint64_t ubr = s.total;
+    ProfScope prof(stats, stats && stats->cur_tag == PROF_ACC_G1 ? PROF_PAIR_G1 : PROF_PAIR_G2, stream);
+    const Affine<F>* src = d_bases; const uint32_t* keys = s.keys; const uint64_t* cin = s.counts;
     for (int r = 0; r < R; r++) {
-        rc = msm_pair_next_offsets(in, NB, sizes, out, base + o_tmp, scan_tmp, stream); launches += 3;
+        uint64_t* cout = (uint64_t*)(base + (size_t)r * 128);
+        const unsigned grid = (unsigned)(T[r] / PAIR_THREADS), igrid = (unsigned)((T[r] / PAIR_LANE_PRODUCTS + 127) / 128);
+        if (r == 0) k_pair_prefix<F, true><<<grid, PAIR_THREADS, 0, stream>>>(src, s.vals, keys, cin, Jub[r], K[r], pre, tprod, outc);
+        else k_pair_prefix<F, false><<<grid, PAIR_THREADS, 0, stream>>>(src, nullptr, keys, cin, Jub[r], K[r], pre, tprod, outc);
+        int rc = msm_pair_scan(outc, pos, Jub[r] + 1, base + o_tmp, scan_tmp, stream);
         if (rc) return rc;
-        ubr = (ubr + NB + 1) / 2;
-        const unsigned grid = (unsigned)(((ubr + PAIR_K - 1) / PAIR_K + PAIR_THREADS - 1) / PAIR_THREADS);
-        if (r == 0) k_pair_round<F, true><<<grid, PAIR_THREADS, 0, stream>>>(src, s.vals, in, out, NB, P[0], K[0], Ls);
-        else k_pair_round<F, false><<<grid, PAIR_THREADS, 0, stream>>>(src, nullptr, in, out, NB, P[r & 1], K[r & 1], Ls);
-        launches++;
-        src = P[r & 1]; s2.keys = K[r & 1];
-        uint32_t* t = in; in = out; out = t;
+        k_pair_invert<F><<<igrid, 128, 0, stream>>>(tprod, T[r], invp, pos, Jub[r], cout, wave);
+        if (r == 0) k_pair_apply<F, true><<<grid, PAIR_THREADS, 0, stream>>>(src, s.vals, keys, cin, K[r], pre, invp, pos, P[0], Kb[0]);
+        else k_pair_apply<F, false><<<grid, PAIR_THREADS, 0, stream>>>(src, nullptr, keys, cin, K[r], pre, invp, pos, P[r & 1], Kb[r & 1]);
+        launches += 5;   // prefix, scan (2), invert, apply
+        src = P[r & 1]; keys = Kb[r & 1]; cin = cout;
     }
-    rc = msm_pair_counts(in, NB, counts2, stream); launches++;
-    if (rc) return rc;
-    s2.counts = counts2;
     prof.end();
     if (stats) stats->launches += launches;
-    // the segmented pipeline on the reduced list; its own accumulate launch is not separately profiled (nev guard)
-    cudaEvent_t* sev = stats ? stats->ev : nullptr; if (stats) stats->ev = nullptr;
-    rc = msm_buckets_impl<F>(src, s2, scratch, o_rest, stream, d_wsum, stats, tail_stream, ev_acc);
-    if (stats) stats->ev = sev;
-    return rc;
+    s2.keys = keys; s2.counts = cin;
+    return msm_buckets_impl<F>(src, s2, scratch, o_rest, stream, d_wsum, stats, tail_stream, ev_acc);
 }
 
 template <class F>
@@ -749,27 +798,20 @@ int msm_buckets_impl(const Affine<F>* d_bases, const MsmSorted& s, MsmScratch& s
     const MsmGeom g = s.g;
     const uint32_t NW = g.windows();
     const uint64_t nbuckets = (uint64_t)NW * g.B;
-    const uint64_t heads0 = (s.total + s.seg_lo - 1) / s.seg_lo;   // upper bound; the device knows the exact count (counts[1])
-    const uint64_t heads1 = (heads0 + MSM_SEG - 1) / MSM_SEG;
     const uint32_t L = g.B < (uint32_t)MSM_RED_CHUNK ? g.B : MSM_RED_CHUNK;
     const uint32_t chunks = g.B / L;
     const uint32_t red_threads = 128;
     const uint32_t ctas_per_window = (chunks + red_threads - 1) / red_threads;
-    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
-    size_t o_buckets = 0;
-    size_t o_headsA = o_buckets + al(nbuckets * sizeof(XYZZ<F>)), o_hkA = o_headsA + al(heads0 * sizeof(XYZZ<F>));
-    size_t o_headsB = o_hkA + al(heads0 * 4), o_hkB = o_headsB + al(heads1 * sizeof(XYZZ<F>));
-    size_t o_hkM = o_hkB + al(heads1 * 4);                     // level-1 keys after the short-run fast path
-    size_t o_part = o_hkM + al(heads0 * 4);
-    size_t bytes = o_part + al(msm_reduce_scratch_elems(g) * sizeof(XYZZ<F>));
-    uint8_t* base = (uint8_t*)scratch.get(scratch_off + bytes);
+    const MsmBucketLayout lay = msm_bucket_layout<F>(g, s.total, s.seg_lo);
+    const uint64_t heads0 = lay.heads0;
+    uint8_t* base = (uint8_t*)scratch.get(scratch_off + lay.bytes);
     if (!base) return (int)cudaErrorMemoryAllocation;
     base += scratch_off;
-    XYZZ<F>* buckets = (XYZZ<F>*)(base + o_buckets);
-    XYZZ<F>* headsA = (XYZZ<F>*)(base + o_headsA); uint32_t* hkA = (uint32_t*)(base + o_hkA);
-    XYZZ<F>* headsB = (XYZZ<F>*)(base + o_headsB); uint32_t* hkB = (uint32_t*)(base + o_hkB);
-    XYZZ<F>* partials = (XYZZ<F>*)(base + o_part);
-    uint32_t* hkM = (uint32_t*)(base + o_hkM);
+    XYZZ<F>* buckets = (XYZZ<F>*)base;
+    XYZZ<F>* headsA = (XYZZ<F>*)(base + lay.headsA); uint32_t* hkA = (uint32_t*)(base + lay.hkA);
+    XYZZ<F>* headsB = (XYZZ<F>*)(base + lay.headsB); uint32_t* hkB = (uint32_t*)(base + lay.hkB);
+    XYZZ<F>* partials = (XYZZ<F>*)(base + lay.part);
+    uint32_t* hkM = (uint32_t*)(base + lay.hkM);
     int launches = 0;
     cudaMemsetAsync(buckets, 0, nbuckets * sizeof(XYZZ<F>), stream);
     if (heads0) {

@@ -44,68 +44,29 @@ __global__ void k_digits(const uint8_t* __restrict__ scalars, uint32_t sbytes, u
     }
 }
 
-// number of valid (non-zero-digit) entries = first index whose sorted key is INVALID; then the entries per accumulation
-// thread: target T, fitted so that the grid is a whole number of waves of `wave` resident threads (MsmSorted comment).
+// number of valid (non-zero-digit) entries = first index whose sorted key is INVALID, then the counts derived from it
 __global__ void k_count_valid(const uint32_t* __restrict__ keys, uint64_t total, uint64_t* __restrict__ out, uint32_t T, uint32_t seg_lo, uint64_t wave) {
     if (blockIdx.x | threadIdx.x) return;
     uint64_t lo = 0, hi = total;
     while (lo < hi) { uint64_t mid = (lo + hi) >> 1; if (keys[mid] == MSM_INVALID_KEY) hi = mid; else lo = mid + 1; }
-    out[0] = lo;
-    uint64_t seg = T;
-    if (wave) {
-        const uint64_t k = (lo + wave * T - 1) / (wave * T);             // waves at the target size
-        if (k && k <= 3) seg = (lo + k * wave - 1) / (k * wave);      // with 4+ waves the partial last wave still saturates the pipe (measured: no gain, more heads)
-        if (seg < seg_lo) seg = seg_lo;
-        if (seg > T) seg = T;
-    }
-    out[MSM_COUNTS_SEG] = seg;
-    // level sizes for the fold cascade: level 0 always emits ceil(M/seg) heads; a level >= 1 with
-    // <= MSM_SEG inputs is the last one (single thread, everything folded into the buckets) and emits none.
-    uint64_t m = (lo + seg - 1) / seg;
-    out[1] = m;
-    for (int l = 2; l < 8; l++) { m = (m <= MSM_SEG) ? 0 : (m + MSM_SEG - 1) / MSM_SEG; out[l] = m; }
+    msm_fill_counts(out, lo, T, seg_lo, wave);
 }
 
+int msm_sm_count() {
+    static int sm_count = 0;
+    if (!sm_count) { int dev = 0; cudaGetDevice(&dev); if (cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sm_count <= 0) sm_count = 148; }
+    return sm_count;
+}
 
-// ---- helpers of the batched-affine pairing rounds (msm_pair.cuh)
-__global__ void k_bucket_offsets(const uint32_t* __restrict__ keys, const uint64_t* __restrict__ counts, uint32_t NB, uint32_t* __restrict__ off) {
-    uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (b > NB) return;
-    const uint64_t M = counts[0];
-    uint64_t lo = 0, hi = M;                 // first index with key >= b
-    while (lo < hi) { uint64_t mid = (lo + hi) >> 1; if (keys[mid] < b) lo = mid + 1; else hi = mid; }
-    off[b] = (uint32_t)lo;
-}
-__global__ void k_halve_sizes(const uint32_t* __restrict__ off, uint32_t NB, uint32_t* __restrict__ sizes) {
-    uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (b > NB) return;
-    sizes[b] = b < NB ? (off[b + 1] - off[b] + 1) / 2 : 0;
-}
-__global__ void k_counts_from_offsets(const uint32_t* __restrict__ off, uint32_t NB, uint64_t* __restrict__ counts) {
-    if (blockIdx.x | threadIdx.x) return;
-    uint64_t m = off[NB];
-    counts[0] = m;
-    m = (m + MSM_SEG - 1) / MSM_SEG; counts[1] = m;
-    for (int l = 2; l < 8; l++) { m = (m <= (uint64_t)MSM_SEG) ? 0 : (m + MSM_SEG - 1) / MSM_SEG; counts[l] = m; }
-    counts[MSM_COUNTS_SEG] = MSM_SEG;
-}
-size_t msm_pair_scan_tmp_bytes(uint32_t NB) {
+// ---- output positions of a batched-affine round (msm_pair.cuh): exclusive sum of the per-slot output counts
+size_t msm_pair_scan_tmp_bytes(uint64_t items) {
     size_t bytes = 0;
-    cub::DeviceScan::ExclusiveSum(nullptr, bytes, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)(NB + 1));
+    cub::DeviceScan::ExclusiveSum(nullptr, bytes, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)items);
     return bytes;
 }
-int msm_pair_offsets(const uint32_t* keys, const uint64_t* counts, uint32_t NB, uint32_t* off, cudaStream_t stream) {
-    k_bucket_offsets<<<(NB + 1 + 255) / 256, 256, 0, stream>>>(keys, counts, NB, off);
-    return (int)cudaGetLastError();
-}
-int msm_pair_next_offsets(const uint32_t* off_in, uint32_t NB, uint32_t* sizes, uint32_t* off_out, void* tmp, size_t tmp_bytes, cudaStream_t stream) {
-    k_halve_sizes<<<(NB + 1 + 255) / 256, 256, 0, stream>>>(off_in, NB, sizes);
-    cudaError_t e = cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, sizes, off_out, (int)(NB + 1), stream);
+int msm_pair_scan(const uint32_t* counts, uint32_t* pos, uint64_t items, void* tmp, size_t tmp_bytes, cudaStream_t stream) {
+    cudaError_t e = cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, counts, pos, (int)items, stream);
     return (int)(e != cudaSuccess ? e : cudaGetLastError());
-}
-int msm_pair_counts(const uint32_t* off, uint32_t NB, uint64_t* counts, cudaStream_t stream) {
-    k_counts_from_offsets<<<1, 1, 0, stream>>>(off, NB, counts);
-    return (int)cudaGetLastError();
 }
 
 int msm_sort_entries(const uint8_t* d_scalars, uint32_t sbytes, uint64_t n, MsmGeom g, MsmScratch& scratch,
@@ -138,9 +99,7 @@ int msm_sort_entries(const uint8_t* d_scalars, uint32_t sbytes, uint64_t n, MsmG
     const bool adaptive = g_msm_tuning[5] >= 0 && g_msm_tuning[7] <= 0;
     if (adaptive) { const uint64_t avg = nbuckets ? total / nbuckets : 0; while (T < 256 && avg > 2ull * T) T <<= 1; }
     if (g_msm_tuning[7] > 0) T = (uint32_t)g_msm_tuning[7];
-    static int sm_count = 0;
-    if (!sm_count) { int dev = 0; cudaGetDevice(&dev); if (cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sm_count <= 0) sm_count = 148; }
-    const uint64_t wave = adaptive ? (uint64_t)sm_count * 4 * MSM_ACC_THREADS : 0;     // 4 CTAs of 128 threads per SM (2 for the extension-field kernels: same fit)
+    const uint64_t wave = adaptive ? (uint64_t)msm_sm_count() * 4 * MSM_ACC_THREADS : 0;     // 4 CTAs of 128 threads per SM (2 for the extension-field kernels: same fit)
     const uint32_t seg_lo = adaptive ? (T == (uint32_t)MSM_SEG ? 16u : T / 2) : T;
     k_count_valid<<<1, 1, 0, stream>>>(kb.Current(), total, counts, T, seg_lo, wave); launches++;
     prof.end();
